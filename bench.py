@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- tokens/sec of one Llama-3-8B training step under a Galvatron per-layer hybrid strategy on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]                      (N > 1: launched under torchrun)
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]  (N > 1: launched under torchrun)
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]     (CPU restatement of the reference path)
 
 One "step" = forward_backward over the global batch (chunks microbatches) + optimizer step, through the public API
@@ -66,7 +66,13 @@ def parse():
     p.add_argument("--total-budget-s", type=float, default=760.0, help="wall-clock budget of the whole bench.py run (legs are skipped beyond it)")
     p.add_argument("--no-probe", action="store_true")
     p.add_argument("--legs-only", action="store_true", help="debug: skip the headline run, run the path legs only (prints {\"path_legs\": ...})")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", default=None, metavar="DIR",
+                   help="after the timed steps, write what the last timed step returned (its loss, a fixed seeded sample of the fp32 "
+                        "master weights its optimizer update wrote) as DIR/<name>.npy, to compare two builds output for output")
+    opts = p.parse_args()
+    if opts.steps < 1:
+        p.error("--steps must be at least 1")
+    return opts
 
 
 def strategy_for(n_gpus, path=None):
@@ -328,6 +334,31 @@ def kernel_breakdown(step_fn, path, ms_per_step):
                    "kernels": [{"name": n, "launches": c, "ms": ms, "share_of_sum": round(ms / total, 4)} for n, c, ms in rows[:60]]}, f, indent=1)
 
 
+DUMP_WEIGHT_BYTES = 48 << 20     # fp32 weight samples of --dump-outputs, all units together (the files stay under 64 MB)
+
+
+def dump_outputs(path, model, loss):
+    """--dump-outputs: what the last timed step handed back to its caller on this rank -- ``loss.npy`` (float64; absent on a
+    pipeline stage without the loss) and, per optimizer-facing parameter (the fp32 flat master of one unit, this rank's shard),
+    ``<name>.npy``: its values at a fixed sample of positions (seed 0, sorted, the whole tensor when it is small enough).
+    The inputs are the same on every run, but the step is not bit-reproducible (the order of some fp32 accumulations varies), so
+    compare with a tolerance: two runs of one build (B200, 1000 W power limit, --steps 2 --warmup 1) gave losses 4e-5 apart (relative)."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    if loss is not None:
+        np.save(os.path.join(path, "loss.npy"), np.array([loss], dtype=np.float64))
+    params = list(model.named_parameters())
+    per_param = DUMP_WEIGHT_BYTES // 4 // max(1, len(params))
+    gen = torch.Generator().manual_seed(0)
+    for name, p in params:
+        flat = p.detach().reshape(-1)
+        if flat.numel() > per_param:
+            idx = torch.randint(flat.numel(), (per_param,), generator=gen).sort().values
+            flat = flat[idx.to(flat.device)]
+        np.save(os.path.join(path, name + ".npy"), flat.float().cpu().numpy())
+
+
 def run_ours(opts):
     os.environ.setdefault("PYTORCH_CUDA_ALLOC_CONF", "expandable_segments:True")   # 150+ GiB of long-lived state: avoid fragmentation
     import torch
@@ -437,6 +468,8 @@ def run_ours(opts):
     prof, be.gemm_profile = be.gemm_profile, None
     ms_e2e, _, loss_e2e = timed(resident=False)
     clocks = sampler.stop() if rank == 0 else None
+    if opts.dump_outputs and rank == 0:
+        dump_outputs(opts.dump_outputs, model, loss_e2e)
     # one more step with every collective bracketed by CUDA events on its own stream: the in-step NVLink roofline
     be.comm_profile = {}
     t, l = host[W]
